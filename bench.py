@@ -275,6 +275,28 @@ def _calibrate(torch, eng, x, lens, offs, target_ms):
     return max(1, int(target_ms / max(per, 1e-3) + 0.999))
 
 
+DUMP_BYTES_PER_ARRAY = 30_000_000  # two arrays: --dump-outputs writes at most 60 MB
+
+
+def dump_outputs(dirname, arrays, seed=0):
+    """Writes `name -> (cuts, T, dim)` feature arrays as DIR/<name>.npy (float32).  Where an array exceeds
+    DUMP_BYTES_PER_ARRAY, a fixed seeded sample of whole cuts (ascending cut order) is written instead, so that the same
+    arguments always select the same cuts."""
+    import numpy as np
+    import torch
+
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        n = a.shape[0]
+        keep = max(1, min(n, DUMP_BYTES_PER_ARRAY // (a[0].numel() * 4 if torch.is_tensor(a) else a[0].nbytes)))
+        idx = np.sort(np.random.RandomState(seed).choice(n, keep, replace=False)) if keep < n else np.arange(n)
+        if torch.is_tensor(a):
+            a = a[torch.from_numpy(idx).to(a.device)].cpu().numpy()
+        else:
+            a = a[idx]
+        np.save(os.path.join(dirname, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def run_b200(args):
     world = int(os.environ.get("WORLD_SIZE", 1))
     nsamp = int(args.cut_seconds * SR)
@@ -368,6 +390,10 @@ def run_b200(args):
     e2e_value = world * (Be * nsamp / SR / 3600.0) * args.e2e_calls * args.e2e_steps / e2e_max
     d2h_bytes = int(feats.size) * 4 * args.e2e_calls
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # every step's first launch reads buffer 0, so outs[0] holds what the last step computed for it whatever the
+        # calibrated launch count; `feats` is the last public-API call's result
+        dump_outputs(args.dump_outputs, {"fbank_device": outs[0].view(B, frames // B, eng.feature_dim), "fbank_e2e": feats})
 
     extra = {}
     if not args.no_extra:
@@ -541,6 +567,10 @@ def main():
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-cutset", action="store_true")
     ap.add_argument("--cutset-hours", type=float, default=4.0, help="hours of audio per rank in the CutSet-level job of `extra`")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's features of the last step as DIR/fbank_device.npy (device-resident "
+                         "leg, input buffer 0) and DIR/fbank_e2e.npy (last extract_batch call), float32 (cuts, frames, 80); a fixed "
+                         "seeded sample of cuts where an array exceeds 30 MB")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -33,6 +33,20 @@ def load_golden_stream():
     return [(i, m, g[f"x{i}"], g[f"y{i}"], g[f"r{i}"]) for i, m in enumerate(meta)]
 
 
+def load_golden_reference_api():
+    """tests/golden/golden_reference_api_v1.npz (make_golden_reference_api.py): (manifest dict, arrays by name)."""
+    g = np.load(os.path.join(os.path.dirname(GOLDEN), "golden_reference_api_v1.npz"))
+    return json.loads(bytes(g["manifest"]).decode()), {k: g[k] for k in g.files if k != "manifest"}
+
+
+def as_config(d):
+    """A reference config stored as a dict, back as an object with the same attributes (kaldifeat's nested options
+    included): `build_plan` reads configs by field name."""
+    from types import SimpleNamespace
+
+    return SimpleNamespace(**{k: as_config(v) if isinstance(v, dict) else v for k, v in d.items()})
+
+
 def oracle_cfg(feature, cfg):
     return O.OracleConfig(feature=feature, **cfg)
 

@@ -12,8 +12,7 @@ import numpy as np
 import pytest
 import torch
 
-import refshim
-from helpers import attach_oracle_engine
+from helpers import attach_oracle_engine, load_golden_reference_api
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -45,36 +44,33 @@ TA_SPEC_GOLD = _ta_spec_golden()
 
 
 # ------------------------------------------------------------------------------------------------ CPU tier
-@pytest.mark.reference
-@pytest.mark.skipif(not refshim.reference_available(), reason="reference tree not present")
 def test_config_surfaces_match_the_reference_field_for_field():
-    refshim.import_reference()
-    from lhotse.features.fbank import TorchaudioFbankConfig
-    from lhotse.features.kaldifeat import (KaldifeatFbankConfig, KaldifeatFrameOptions, KaldifeatMelOptions,
-                                           KaldifeatMfccConfig)
-    from lhotse.features.mfcc import TorchaudioMfccConfig
-    from lhotse.features.spectrogram import TorchaudioSpectrogramConfig
-
+    """Against the reference's config dataclasses as stored in tests/golden/golden_reference_api_v1.npz: field names,
+    default values and `to_dict()` output."""
+    man, _ = load_golden_reference_api()
+    ref = man["config_surfaces"]
     _, fam = _lb()
-    pairs = [(TorchaudioFbankConfig, fam.B200TorchaudioFbankConfig), (TorchaudioMfccConfig, fam.B200TorchaudioMfccConfig),
-             (TorchaudioSpectrogramConfig, fam.B200TorchaudioSpectrogramConfig),
-             (KaldifeatFrameOptions, fam.B200KaldifeatFrameOptions), (KaldifeatMelOptions, fam.B200KaldifeatMelOptions),
-             (KaldifeatFbankConfig, fam.B200KaldifeatFbankConfig), (KaldifeatMfccConfig, fam.B200KaldifeatMfccConfig)]
-    for ref_cls, our_cls in pairs:
+    pairs = [("TorchaudioFbankConfig", fam.B200TorchaudioFbankConfig), ("TorchaudioMfccConfig", fam.B200TorchaudioMfccConfig),
+             ("TorchaudioSpectrogramConfig", fam.B200TorchaudioSpectrogramConfig),
+             ("KaldifeatFrameOptions", fam.B200KaldifeatFrameOptions), ("KaldifeatMelOptions", fam.B200KaldifeatMelOptions),
+             ("KaldifeatFbankConfig", fam.B200KaldifeatFbankConfig), ("KaldifeatMfccConfig", fam.B200KaldifeatMfccConfig)]
+    assert sorted(ref) == sorted(name for name, _ in pairs)
+    for ref_name, our_cls in pairs:
         ours = {f.name: f for f in dataclasses.fields(our_cls)}
-        ref_inst, our_inst = ref_cls(), our_cls()
-        for f in dataclasses.fields(ref_cls):
-            assert f.name in ours, (ref_cls.__name__, f.name)
-            if f.name in ("device", "frame_opts", "mel_opts"):
+        ref_fields, ref_defaults = ref[ref_name]["fields"], ref[ref_name]["defaults"]
+        our_inst = our_cls()
+        for name in ref_fields:
+            assert name in ours, (ref_name, name)
+            if name in ("device", "frame_opts", "mel_opts"):
                 continue
-            assert getattr(ref_inst, f.name) == getattr(our_inst, f.name), (ref_cls.__name__, f.name)
-        extra = set(ours) - {f.name for f in dataclasses.fields(ref_cls)}
+            assert json.loads(json.dumps(getattr(our_inst, name))) == ref_defaults[name], (ref_name, name)
+        extra = set(ours) - set(ref_fields)
         assert extra <= {"device", "kernel"}, (our_cls.__name__, extra)
         # a dict written by the reference loads into ours
-        loaded = our_cls.from_dict(ref_inst.to_dict())
+        loaded = our_cls.from_dict(dict(ref[ref_name]["to_dict"]))
         assert dataclasses.asdict(loaded) == dataclasses.asdict(dataclasses.replace(our_inst, **(
-            {"device": "cpu"} if "device" in {f.name for f in dataclasses.fields(ref_cls)} else {})))
-    assert fam.B200KaldifeatFrameOptions().to_dict() == KaldifeatFrameOptions().to_dict()  # ms / samp_freq spelling
+            {"device": "cpu"} if "device" in ref_fields else {})))
+    assert fam.B200KaldifeatFrameOptions().to_dict() == ref["KaldifeatFrameOptions"]["to_dict"]  # ms / samp_freq spelling
 
 
 def test_family_registry_names_and_round_trips(tmp_path):

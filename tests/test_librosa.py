@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-import refshim
+from helpers import load_golden_reference_api
 from lhotse_b200 import build_plan
 from lhotse_b200.plan import PAD_CENTER, make_periodic_window, make_slaney_mel_bank
 from oracle import librosa_oracle as LO
@@ -57,23 +57,20 @@ def test_librosa_oracle_matches_golden(i, c, x, y):
     assert ok, msg
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not refshim.reference_available(), reason="reference tree not present")
 def test_librosa_oracle_against_live_reference_on_the_standin():
-    pytest.importorskip("transformers")
-    refshim.install_librosa_standin()
-    refshim.import_reference()
-    from lhotse.features.librosa_fbank import LibrosaFbank, LibrosaFbankConfig
+    """Against the reference's `LibrosaFbank.extract` (run on the stand-in) on the same seeded inputs, stored by
+    tests/golden/make_golden_reference_api.py."""
+    from golden.make_golden_reference_api import librosa_inputs
 
-    rs = np.random.RandomState(77)
-    for over in ({}, dict(sampling_rate=16000, fft_size=512, hop_size=160, fmin=0, fmax=8000)):
-        cfg = LibrosaFbankConfig(**over)
-        for n in (cfg.fft_size // 2 + 1, 5000, 22051):
-            x = (0.2 * rs.randn(n)).astype(np.float32)
-            want = LibrosaFbank(cfg).extract(x, cfg.sampling_rate)
-            got = LO.extract(x, **cfg.to_dict())
-            assert got.shape == want.shape
-            np.testing.assert_allclose(got, want, rtol=0, atol=2e-5)
+    man, arr = load_golden_reference_api()
+    cfgs = man["librosa_configs"]
+    cases = list(librosa_inputs(cfgs))
+    assert [(c["config"], c["n"]) for c in man["librosa"]] == [(k, n) for k, n, _ in cases] and len(cases) == 6
+    for j, (k, n, x) in enumerate(cases):
+        want = arr[f"librosa{j}"]
+        got = LO.extract(x, **cfgs[k])
+        assert got.shape == want.shape
+        np.testing.assert_allclose(got, want, rtol=0, atol=2e-5)
 
 
 def test_librosa_tables_pinned():

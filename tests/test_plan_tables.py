@@ -1,11 +1,11 @@
 """Constant tables built by the product (lhotse_b200/plan.py) are bit-identical to the oracle's
-(and, in the build container, to the reference module parameters)."""
+and to the reference module parameters (stored golden data)."""
 import math
 
 import numpy as np
 import pytest
 
-import refshim
+from helpers import as_config, load_golden_reference_api
 from lhotse_b200 import (B200Fbank, B200FbankConfig, B200LogSpectrogramConfig, B200Mfcc, B200MfccConfig,
                          B200Spectrogram, B200SpectrogramConfig, build_plan)
 from lhotse_b200.plan import make_window
@@ -80,31 +80,25 @@ def test_plan_dims_and_validation():
     assert np.array_equal(q.window, p.window) and np.array_equal(q.mel_bank, p.mel_bank)
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not refshim.reference_available(), reason="reference tree not present")
 def test_tables_equal_live_reference_and_foreign_configs():
-    refshim.import_reference()
-    from lhotse.features.fbank import TorchaudioFbankConfig
-    from lhotse.features.kaldi.extractors import Fbank, FbankConfig, Mfcc, MfccConfig
-    from lhotse.features.kaldifeat import KaldifeatFbankConfig, KaldifeatMfccConfig
-    from lhotse.features.mfcc import TorchaudioMfccConfig
-
-    for kw in CASES[:7]:
-        ref = Fbank(FbankConfig(**kw)).extractor
-        plan = build_plan("fbank", FbankConfig(**kw))  # the reference's own config object is accepted
-        assert np.array_equal(plan.mel_bank, ref._fb.detach().numpy())
-        assert np.array_equal(plan.window, ref.wav2win._window.detach().numpy())
-    ref = Mfcc(MfccConfig()).extractor
-    plan = build_plan("mfcc", MfccConfig())
-    assert np.array_equal(plan.dct, ref._dct.numpy()) and np.array_equal(plan.lifter, ref._lifter.numpy())
+    """Against the reference module parameters and config objects stored in tests/golden/golden_reference_api_v1.npz."""
+    man, arr = load_golden_reference_api()
+    assert len(man["fbank_configs"]) == 7 and all(man["fbank_configs"][i][k] == v for i, kw in enumerate(CASES[:7]) for k, v in kw.items())
+    for i, d in enumerate(man["fbank_configs"]):
+        plan = build_plan("fbank", as_config(d))  # the reference's own config fields are accepted
+        assert np.array_equal(plan.mel_bank, arr[f"fbank{i}_mel_bank"])
+        assert np.array_equal(plan.window, arr[f"fbank{i}_window"])
+    plan = build_plan("mfcc", as_config(man["mfcc_config"]))
+    assert np.array_equal(plan.dct, arr["mfcc_dct"]) and np.array_equal(plan.lifter, arr["mfcc_lifter"])
     # torchaudio / kaldifeat config families normalise onto the same plan
-    p = build_plan("fbank", TorchaudioFbankConfig())
+    fam = {k: as_config(v) for k, v in man["family_configs"].items()}
+    p = build_plan("fbank", fam["TorchaudioFbankConfig"])
     assert (p.L, p.S, p.N, p.num_filters, p.preemph_coeff, p.energy_style) == (400, 160, 512, 80, 0.97, 1)
-    p = build_plan("mfcc", TorchaudioMfccConfig())
+    p = build_plan("mfcc", fam["TorchaudioMfccConfig"])
     assert (p.num_filters, p.num_ceps) == (23, 13)
-    p = build_plan("fbank", KaldifeatFbankConfig())
+    p = build_plan("fbank", fam["KaldifeatFbankConfig"])
     assert (p.L, p.S, p.N, p.num_filters, p.snip_edges) == (400, 160, 512, 80, False)
-    p = build_plan("mfcc", KaldifeatMfccConfig())
+    p = build_plan("mfcc", fam["KaldifeatMfccConfig"])
     assert (p.num_filters, p.num_ceps) == (23, 13) and math.isclose(p.lifter[1], 1 + 11 * math.sin(math.pi / 22), rel_tol=1e-6)
 
 

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-import refshim
+from helpers import load_golden_reference_api
 from lhotse_b200 import LOG_EPSILON, build_plan
 from lhotse_b200.plan import PAD_CENTER, make_slaney_mel_bank
 from oracle import whisper_oracle as W
@@ -59,24 +59,20 @@ def test_whisper_oracle_matches_golden(i, c, x, y):
     np.testing.assert_allclose(got, y, rtol=0, atol=2e-6)
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not refshim.reference_available(), reason="reference tree not present")
 def test_whisper_oracle_bit_identical_to_live_reference():
-    pytest.importorskip("transformers")
-    refshim.install_librosa_standin()
-    refshim.import_reference()
-    from lhotse.features.whisper_fbank import WhisperFbank, WhisperFbankConfig
+    """Against the reference's `WhisperFbank.extract` on the same seeded inputs, stored by
+    tests/golden/make_golden_reference_api.py."""
+    from golden.make_golden_reference_api import whisper_inputs
 
-    rs = np.random.RandomState(123)
-    for M in (80, 128):
-        ref = WhisperFbank(WhisperFbankConfig(num_filters=M))
-        for n in (640, 4000, 16000, 16080, 31999):
-            x = (0.2 * rs.randn(n)).astype(np.float32)
-            want = ref.extract(x, 16000)
-            got = W.extract(x, M)
-            assert got.shape == want.shape
-            assert np.array_equal(got, want), (M, n, np.abs(got - want).max())
-            assert np.array_equal(W.extract(x[None, :], M), want)  # (1, n) input
+    man, arr = load_golden_reference_api()
+    cases = list(whisper_inputs())
+    assert [(c["num_filters"], c["n"]) for c in man["whisper"]] == [(M, n) for M, n, _ in cases]
+    for j, (M, n, x) in enumerate(cases):
+        want = arr[f"whisper{j}"]
+        got = W.extract(x, M)
+        assert got.shape == want.shape
+        assert np.array_equal(got, want), (M, n, np.abs(got - want).max())
+        assert np.array_equal(W.extract(x[None, :], M), want)  # (1, n) input
 
 
 def test_mel_table_pinned_to_transformers():
